@@ -10,7 +10,11 @@ latents).  `value` times device-resident inputs; `e2e` times the public API
 (ns2vc_b200.api.sample_latents) from pinned host tensors to a host result, copies inside the timed
 region.  Weak scaling over GPUs (independent utterances per rank, SURVEY.md §8e).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+--dump-outputs DIR writes the final latents of the last timed step of both paths, [world x B, 100, T]
+float32: DIR/latents.npy (`value`'s path) and DIR/latents_e2e.npy (`e2e`'s path).  Weights and inputs
+are seeded, so the same arguments give the same inputs on every run.
+
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 """
 from __future__ import annotations
 
@@ -296,6 +300,21 @@ def ncu_traffic(kernel):
     return tot / n if n else None
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def write_dumps(path, arrays):
+    """Write each tensor as float32 ``path/<name>.npy``; refuse rather than write more than DUMP_LIMIT_BYTES in all."""
+    import numpy as np
+    arrays = {k: v.detach().to("cpu", torch.float32).numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT_BYTES:
+        raise SystemExit(f"--dump-outputs: {total} bytes of outputs exceed the {DUMP_LIMIT_BYTES}-byte limit")
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, f"{k}.npy"), a)
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -303,7 +322,14 @@ def main():
     ap.add_argument("--warmup", type=int, default=3)
     ap.add_argument("--impl", default="b200")
     ap.add_argument("--nfe", type=int, default=NFE, help=argparse.SUPPRESS)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the latents of the last timed step as DIR/<name>.npy (float32) "
+                         "so two builds can be compared output for output; the inputs are seeded")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs applies to the b200 path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local = int(os.environ.get("LOCAL_RANK", "0"))
@@ -348,6 +374,7 @@ def main():
         out = sess.sample_dpmpp_2m(x_d, ns, ts)
         if world > 1:
             gather_latents(out, out=gathered)
+            return gathered
         return out
 
     def run_e2e():
@@ -368,7 +395,7 @@ def main():
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(K):
-            fn()
+            last = fn()
         e1.record()
         torch.cuda.synchronize(dev)
         clocks = cs.stop() if cs else None
@@ -377,9 +404,10 @@ def main():
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
-        return float(ms.item()), clocks
+        return float(ms.item()), clocks, last
 
-    ms, clocks = timed(run_device, args.steps, args.warmup, sample_clocks=True)
+    ms, clocks, last = timed(run_device, args.steps, args.warmup, sample_clocks=True)
+    dumps = {"latents": last.cpu()} if args.dump_outputs and rank == 0 else {}
     # kernel launches per run, counted from the engine's own launch programs (one memset node per
     # forward is not a kernel and is subtracted; +1 sampler-update kernel per step)
     cnt = DenoiserSession(unet, content_d, prompt_d, mask_d)
@@ -391,7 +419,10 @@ def main():
     del cnt
     units = world * B * nfe * args.steps
     value = units / (ms / 1e3)
-    ms_e2e, _ = timed(run_e2e, args.steps, 1)
+    ms_e2e, _, last = timed(run_e2e, args.steps, 1)
+    if args.dump_outputs and rank == 0:
+        dumps["latents_e2e"] = last
+        write_dumps(args.dump_outputs, dumps)
     e2e_val = units / (ms_e2e / 1e3)
     h2d = sum(hin[k].numel() * hin[k].element_size() for k in ("x", "content", "prompt", "refer_lengths"))
     d2h = (world if rank == 0 else 1) * B * 100 * T * 4

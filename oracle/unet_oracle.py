@@ -72,7 +72,7 @@ def text_time_embedding(sd, p: str, ehs: torch.Tensor, num_heads: int) -> torch.
     v = shape(F.linear(x, sd[p + ".pool.v_proj.weight"], sd[p + ".pool.v_proj.bias"]))
     scale = 1 / math.sqrt(math.sqrt(dph))
     weight = torch.einsum("bct,bcs->bts", q * scale, k * scale)
-    weight = torch.softmax(weight.float(), dim=-1)
+    weight = torch.softmax(weight.float(), dim=-1).type(weight.dtype)
     a = torch.einsum("bts,bcs->bct", weight, v)
     a = a.reshape(bs, -1, 1).transpose(1, 2)[:, 0, :]
     a = F.linear(a, sd[p + ".proj.weight"], sd[p + ".proj.bias"])

@@ -1,55 +1,59 @@
-"""Drop-in check against the real reference tree (only where /root/reference exists: the build
-container).  `ns2vc_b200.install()` + the reference's own model.py must construct, expose the same
-state_dict contract, and strict-load a reference-shaped checkpoint."""
-import json
-import os
+"""Drop-in check against what the reference's own model.py builds (tests/golden/reference_model.pt, recorded from the unmodified
+reference by oracle/make_golden_dropin.py).  After `ns2vc_b200.install()` / `install_pre_model()` the names model.py imports
+resolve to the B200 classes, and those classes, built with model.py's arguments, expose the reference's state_dict contract
+and strict-load a reference-shaped checkpoint."""
+import importlib
 import sys
-from unittest.mock import MagicMock
+import types
 
-import pytest
 import torch
 
-REF = os.environ.get("NS2VC_REFERENCE", "/root/reference")
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, "unet1d")), reason="reference tree not present")
 
-
-def test_reference_model_py_builds_on_our_unet():
+def test_reference_model_py_builds_on_our_unet(gold):
     import ns2vc_b200
-    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] in ("unet1d", "sampler", "model", "modules", "utils", "operations")}
-    for k in saved:
-        del sys.modules[k]
-    sys.path.insert(0, REF)
+    from ns2vc_b200 import dpm_solver, uni_pc, unet as unet_mod
+    from ns2vc_b200.arch import ns2vc_denoiser_config, param_shapes
+    from ns2vc_b200.pre_model import Pre_model
+    from ns2vc_b200.unet import UNet1DConditionModel
+    g = gold("reference_model.pt")
+    cfg = g["config"]
+
+    # every name model.py imports from the aliased modules resolves to ours
+    saved = {k: v for k, v in sys.modules.items() if k.split(".")[0] in ("unet1d", "sampler")}
     try:
-        for name in ("matplotlib", "matplotlib.pyplot", "vocos", "accelerate", "librosa", "soundfile", "tensorboardX"):
-            sys.modules.setdefault(name, MagicMock())
         ns2vc_b200.install()
-        import model as ref_model
-        from ns2vc_b200.unet import UNet1DConditionModel
-        cfg = json.load(open(os.path.join(REF, "config.json")))
-        ref_pre_keys = {k: tuple(v.shape) for k, v in ref_model.Pre_model(cfg).state_dict().items()}   # the reference's own class
-        ns2vc_b200.install_pre_model(ref_model)
-        ns2 = ref_model.NaturalSpeech2(cfg)
-        from ns2vc_b200.pre_model import Pre_model
-        assert isinstance(ns2.pre_model, Pre_model)
-        ours = {k: tuple(v.shape) for k, v in ns2.pre_model.state_dict().items()}
-        assert list(ours.items()) == list(ref_pre_keys.items())          # same keys, order and shapes as the reference's Pre_model
-        assert sum(p.numel() for p in ns2.pre_model.parameters()) == 34923404
-        unet = ns2.diff_model.unet
-        assert isinstance(unet, UNet1DConditionModel)
-        assert sum(p.numel() for p in unet.parameters()) == 66076900
-        assert unet.latent_channels == cfg["diffusion_encoder"]["in_channels"]
-        # a checkpoint written by the reference has exactly these keys under diff_model.unet.
-        from ns2vc_b200.arch import ns2vc_denoiser_config, param_shapes
-        keys = [k for k in ns2.state_dict() if k.startswith("diff_model.unet.")]
-        assert [k[len("diff_model.unet."):] for k in keys] == list(param_shapes(ns2vc_denoiser_config()).keys())
-        ns2.load_state_dict(ns2.state_dict(), strict=True)
-        from sampler.dpm_solver import DPM_Solver
-        from sampler.uni_pc import UniPC
-        from ns2vc_b200 import dpm_solver, uni_pc
-        assert DPM_Solver is dpm_solver.DPM_Solver and UniPC is uni_pc.UniPC
+        ours = {"unet1d.unet_1d_condition": unet_mod, "sampler.dpm_solver": dpm_solver, "sampler.uni_pc": uni_pc}
+        assert set(g["imports"]) == set(ours)
+        for mod, names in g["imports"].items():
+            assert names and importlib.import_module(mod) is ours[mod]
+            for name in names:
+                assert getattr(importlib.import_module(mod), name) is getattr(ours[mod], name), (mod, name)
     finally:
-        sys.path.remove(REF)
         for k in list(sys.modules):
-            if k.split(".")[0] in ("unet1d", "sampler", "model", "modules", "utils", "operations"):
+            if k.split(".")[0] in ("unet1d", "sampler"):
                 del sys.modules[k]
         sys.modules.update(saved)
+
+    # model.py:451 looks Pre_model up by its global name
+    model_py = types.ModuleType("model")
+    model_py.Pre_model = object
+    ns2vc_b200.install_pre_model(model_py)
+    assert model_py.Pre_model is Pre_model
+    pre = model_py.Pre_model(cfg)
+    assert [(k, tuple(v.shape)) for k, v in pre.state_dict().items()] == g["pre_model_shapes"]   # keys, order, shapes
+    assert sum(p.numel() for p in pre.parameters()) == g["pre_model_params"] == 34923404
+
+    # Diffusion_Encoder's constructor call (model.py:391-400)
+    unet = UNet1DConditionModel(**g["unet_kwargs"])
+    assert sum(p.numel() for p in unet.parameters()) == g["unet_params"] == 66076900
+    assert unet.latent_channels == cfg["diffusion_encoder"]["in_channels"]
+
+    # a checkpoint written by the reference: its diff_model.unet. and pre_model. entries are exactly our state_dicts
+    ckpt = g["checkpoint_shapes"]
+    unet_keys = [(k[len("diff_model.unet."):], s) for k, s in ckpt if k.startswith("diff_model.unet.")]
+    assert unet_keys == [(k, tuple(v.shape)) for k, v in unet.state_dict().items()]
+    assert [k for k, _ in unet_keys] == list(param_shapes(ns2vc_denoiser_config()).keys())
+    assert [(k[len("pre_model."):], s) for k, s in ckpt if k.startswith("pre_model.")] == g["pre_model_shapes"]
+    assert not [k for k, _ in ckpt if k.startswith("diff_model.") and not k.startswith("diff_model.unet.")]
+    unet.load_state_dict({k: torch.zeros(s) for k, s in unet_keys}, strict=True)
+    pre.load_state_dict({k: torch.zeros(s) for k, s in g["pre_model_shapes"]}, strict=True)
